@@ -20,8 +20,13 @@ One "step" = one pass over the batch of one GPU.
           after the other; with CPUs to spare each decoder also parses ahead on worker threads (edge264_alloc n_threads).
   --impl reference   the reference decoder compiled from its own sources (oracle/_ref), one single-threaded decoder per
           stream on all usable host cores, same streams, same application loop.
+  --dump-outputs DIR  after the timed steps, what the decode loop handed to the application in its last timed step (the
+          kernel-only replay re-runs the kernels of exactly these pictures): a fixed, seeded choice of output frames
+          (DUMP_FRAMES at most) and of sample positions in them, so that two builds can be compared output for output.
+            DIR/frames.npy      float32 [frames, positions]: 8-bit samples of the cropped Y, Cb and Cr planes laid end to end
+            DIR/frame_info.npy  float64 [frames, 7]: unit, index in output order, FrameId, width_Y, height_Y, width_C, height_C
 """
-import argparse, ctypes, json, os, subprocess, sys, threading, time
+import argparse, ctypes, hashlib, json, os, subprocess, sys, tempfile, threading, time
 
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -44,16 +49,24 @@ def generate_streams(cfg, seeds, frames, workdir):
     gen = os.path.join(ROOT, "tools", "gen264")
     if not os.path.exists(gen):
         raise SystemExit("tools/gen264 missing: run `python -c 'import __graft_entry__ as g; g.build()'` first")
+    # a cached stream is named after the generator binary and its arguments and appears only once complete, so the inputs
+    # are what this build's generator writes for these arguments, never a file of another build or of an interrupted run
+    key = hashlib.sha1(open(gen, "rb").read() + cfg["gen"].encode()).hexdigest()[:12]
     procs, paths = [], []
+    def finish(procs):
+        for q, part, p in procs:
+            if q.wait() != 0:
+                raise SystemExit(f"bench.py: tools/gen264 failed on {p}")
+            os.replace(part, p)
     for s in seeds:
-        p = os.path.join(workdir, f"{cfg['w']}x{cfg['h']}_{s}_{frames}.264")
+        p = os.path.join(workdir, f"{cfg['w']}x{cfg['h']}_{s}_{frames}_{key}.264")
         paths.append(p)
         if not os.path.exists(p):
-            procs.append(subprocess.Popen([gen, "-o", p, "-W", str(cfg["w"]), "-H", str(cfg["h"]), "-n", str(frames), "-s", str(s)] + cfg["gen"].split(), stderr=subprocess.DEVNULL))
+            part = f"{p}.{os.getpid()}.part"
+            procs.append((subprocess.Popen([gen, "-o", part, "-W", str(cfg["w"]), "-H", str(cfg["h"]), "-n", str(frames), "-s", str(s)] + cfg["gen"].split(), stderr=subprocess.DEVNULL), part, p))
         if len(procs) >= 16:
-            for q in procs: q.wait()
-            procs = []
-    for q in procs: q.wait()
+            finish(procs); procs = []
+    finish(procs)
     return [open(p, "rb").read() for p in paths]
 
 
@@ -87,6 +100,48 @@ class BenchLib:
         return secs, list(frames), list(sums), decs
 
     def free(self, decs): self.lib.e264bench_free(decs, len(decs))
+
+
+DUMP_FRAMES, DUMP_FLOATS, DUMP_SEED = 32, 15 << 20, 264      # --dump-outputs: at most 60 MB of float32 samples
+
+
+def dump_selection(frames):
+    """The output frames --dump-outputs keeps, given the frame count of every unit: a seeded choice of at most DUMP_FRAMES
+    of them, as (unit, index in output order)."""
+    import numpy as np
+    total = sum(frames)
+    flat = np.sort(np.random.default_rng(DUMP_SEED).choice(total, min(DUMP_FRAMES, total), replace=False))
+    starts = np.cumsum([0] + list(frames[:-1]))
+    unit = np.searchsorted(starts, flat, side="right") - 1
+    return unit.astype(np.int32), (flat - starts[unit]).astype(np.int64)
+
+
+class Capture:
+    """--dump-outputs: the selected output frames are copied by the decode loop itself (e264bench_capture) while the
+    capture is on; write() stores a seeded choice of sample positions of them."""
+    def __init__(self, bench, frames, cfg):
+        import numpy as np
+        # bound here, not in BenchLib: a driver library built before the capture existed still serves every other use
+        if not hasattr(bench.lib, "e264bench_capture"):
+            raise SystemExit(f"bench.py --dump-outputs: {bench.lib._name} has no e264bench_capture; rebuild it from tools/e264_bench.c")
+        bench.lib.e264bench_capture.argtypes = [ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_size_t, ctypes.c_void_p]
+        self.bench, self.unit, self.index = bench, *dump_selection(frames)
+        n, cap = len(self.unit), cfg["w"] * cfg["h"] * 384
+        self.buf = np.zeros((n, cap), np.uint8); self.info = np.full((n, 5), -1, np.int32)
+        self.dst = (ctypes.c_void_p * n)(*[self.buf[k].ctypes.data for k in range(n)])
+        bench.lib.e264bench_capture(n, self.unit.ctypes.data, self.index.ctypes.data, self.dst, cap, self.info.ctypes.data)
+
+    def stop(self):
+        self.bench.lib.e264bench_capture(0, None, None, None, 0, None)
+
+    def write(self, out):
+        import numpy as np
+        assert (self.info[:, 0] >= 0).all(), "a frame chosen for --dump-outputs was not delivered"
+        size = int(min(wy * hy + 2 * wc * hc for _, wy, hy, wc, hc in self.info))
+        pos = np.sort(np.random.default_rng(DUMP_SEED + 1).choice(size, min(size, DUMP_FLOATS // len(self.unit)), replace=False))
+        os.makedirs(out, exist_ok=True)
+        np.save(os.path.join(out, "frames.npy"), self.buf[:, pos].astype(np.float32))
+        np.save(os.path.join(out, "frame_info.npy"), np.column_stack([self.unit, self.index, self.info]).astype(np.float64))
 
 
 class ReplayStats(ctypes.Structure):
@@ -185,11 +240,16 @@ def reference_arm(args, cfg, rank, world, emit):
     n_units = args.streams * world
     bufs = batch_for(cfg, n_units, args.workdir, args.frames)
     threads = max(1, min(usable_cpus(), n_units))   # one single-threaded decoder per usable CPU (cgroup quota respected)
-    for _ in range(args.warmup): ref.run(bufs, threads)
-    t = 0.0; frames = 0
-    for _ in range(args.steps):
+    fr = None
+    for _ in range(args.warmup): _, fr, _, _ = ref.run(bufs, threads)
+    t = 0.0; frames = 0; cap = None
+    for step in range(args.steps):
+        if args.dump_outputs and step == args.steps - 1:
+            cap = Capture(ref, fr or ref.run(bufs, threads)[1], cfg)      # the choice needs every unit's frame count
         s, fr, _, _ = ref.run(bufs, threads)
         t += s; frames += sum(fr)
+    if cap is not None:
+        cap.stop(); cap.write(args.dump_outputs)
     fps = frames / t
     mbpf = cfg["w"] * cfg["h"]
     line = {"metric": cfg["metric"], "value": fps, "unit": "frames/s", "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
@@ -212,7 +272,8 @@ def main():
     ap.add_argument("--streams", type=int, default=0, help="sharding units (streams or GOPs) per GPU; 0 = the config's default")
     ap.add_argument("--frames", type=int, default=0, help="frames per unit; 0 = the config's default")
     ap.add_argument("--dec-threads", type=int, default=-1, help="edge264_alloc n_threads of every decoder; -1 = from the CPUs available per stream")
-    ap.add_argument("--workdir", default=os.environ.get("E264_BENCH_DIR", "/tmp/e264_bench"))
+    ap.add_argument("--workdir", default=os.environ.get("E264_BENCH_DIR", os.path.join(tempfile.gettempdir(), f"e264_bench_{os.getuid()}")))
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a seeded sample of the last timed step's output frames to DIR (see the module docstring)")
     args = ap.parse_args()
     cfg = CONFIGS[args.config]
     if args.streams <= 0: args.streams = cfg["streams"]
@@ -277,12 +338,16 @@ def main():
     frames_per_step = sum(frames)
     sampler = ClockSampler(local); sampler.start()
     barrier()
-    e2e_secs = 0.0
-    for _ in range(args.steps):
+    e2e_secs = 0.0; cap = None
+    for step in range(args.steps):
+        if args.dump_outputs and rank == 0 and step == args.steps - 1:
+            cap = Capture(lib, frames, cfg)
         s, fr, sm, d = lib.run(bufs, app_threads)      # every decoder is freed as soon as its stream ends, like an application would
         lib.free(d)
         e2e_secs += s
         assert sm == sums, "e2e output differs between runs"
+    if cap is not None:
+        cap.stop()
     barrier()
     e2e_secs = maxreduce(e2e_secs)
     e2e_fps = world * frames_per_step * args.steps / e2e_secs
@@ -347,6 +412,8 @@ def main():
                     "note": "edge264_decode_NAL/get_frame from host buffers; bound by the host's CPUs (bitstream parsing) as soon as application threads x (1 + parse-ahead workers) reach the usable CPUs — on one host that is already the case at N = 1, so e2e follows the CPUs, not the number of GPUs; get_frame polls and only waits after ENOBUFS / at the end of a stream"},
             "roofline": roof}
     lib.free(decs)
+    if cap is not None:
+        cap.write(args.dump_outputs)
 
     if rank == 0 and world == 1:
         refp = os.path.join(ROOT, "oracle", "_ref", "libe264bench_ref.so")

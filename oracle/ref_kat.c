@@ -11,6 +11,9 @@
  *                    transform_size_8x8_flag, smooth and noisy pictures
  *   ref_kat dump     prints the known-answer inputs/outputs of the reference's KAT setup as JSON
  *                    (tests/golden/kat_*.json are generated from this)
+ *   ref_kat <fuzz|residual|deblock> --digests FILE   also writes one FNV-1a digest of the reference's outputs per trial
+ *                    (uint32, little-endian) to FILE: tests/golden/kat_fuzz_*.bin, which tests/native/kat_fuzz_check.c
+ *                    replays against the restatement where the reference is not available
  * Nothing from the reference is copied: the sources are compiled from $(REF)/src at build time. */
 #include <stdio.h>
 #include <stdlib.h>
@@ -38,12 +41,17 @@ void port_deblock_chroma_line(uint8_t *pix, int step, int bs, int alpha, int bet
 static uint64_t rs = 88172645463325252ull;
 static unsigned rnd(void) { rs ^= rs << 13; rs ^= rs >> 7; rs ^= rs << 17; return (unsigned)(rs >> 11); }
 
+static FILE *digests;
+static uint32_t fnv(uint32_t h, const void *p, size_t n) { const uint8_t *b = (const uint8_t *)p; for (size_t i = 0; i < n; i++) h = (h ^ b[i]) * 16777619u; return h; }
+static void put_digest(uint32_t d) { if (digests) fwrite(&d, 4, 1, digests); }
+
 static int fuzz_inter(void) {
 	static uint8_t src[64 * 64] __attribute__((aligned(16))), dst[16 * 16] __attribute__((aligned(16)));
 	int bad = 0;
 	for (int trial = 0; trial < 3000 && bad < 10; trial++) {
 		int kind = trial % 4;
 		int px = 1 + rnd() % 3, py = 1 + rnd() % 3, ph = rnd();
+		uint32_t d = 2166136261u;
 		for (int i = 0; i < 64 * 64; i++) src[i] = kind == 0 ? rnd() : kind == 1 ? ((rnd() & 1) ? 255 : 0) : kind == 2 ? (uint8_t)((((i % 64) / px + (i / 64) / py + ph) & 1) ? 255 - rnd() % 3 : rnd() % 3) : ((rnd() % 5) ? 255 : rnd());
 		for (int mode = 0; mode < 48; mode++) {
 			int w = 4 << (mode >> 4), fx = mode & 3, fy = (mode >> 2) & 3;
@@ -52,6 +60,7 @@ static int fuzz_inter(void) {
 				if ((w == 4 && h == 16) || (w == 16 && h == 4)) continue;
 				memset(dst, 0, sizeof(dst));
 				decode_inter_luma(mode, h, 64, src + 20 * 64 + 20, 16, dst, (i8x16){0, 1});
+				for (int y = 0; y < h; y++) d = fnv(d, dst + y * 16, w);
 				Plane P = {src, 64, 64, 64};
 				for (int y = 0; y < h; y++) for (int x = 0; x < w; x++) {
 					int v = port_mc_luma_sample(&P, 20 + x, 20 + y, fx, fy);
@@ -59,6 +68,7 @@ static int fuzz_inter(void) {
 				}
 			}
 		}
+		put_digest(d);
 	}
 	printf("inter luma fuzz: %s\n", bad ? "MISMATCHES" : "ok");
 	return bad;
@@ -94,6 +104,7 @@ static int fuzz_residual(void) {
 		}
 		if (dcidx >= 0) ctx.c[16 + dcidx] = dcv;
 		add_idct4x4(&ctx, iY, dcidx, pix + 32 * 4 + 8);
+		uint32_t d = fnv(2166136261u, pix, sizeof(pix));
 		port_idct4x4(lv, sc, qp, dcidx >= 0, dcv, res);
 		for (int y = 0; y < 4; y++) for (int x = 0; x < 4; x++) want[32 * (4 + y) + 8 + x] = (uint8_t)clip8((int16_t)(want[32 * (4 + y) + 8 + x] + res[y * 4 + x]));
 		if (memcmp(want, pix, sizeof(pix))) { if (bad++ < 5) printf("IDCT4x4 MISMATCH trial %d qp %d plane %d inter %d dcidx %d\n", trial, qp, iY, inter, dcidx); memcpy(want, pix, sizeof(pix)); }
@@ -106,6 +117,7 @@ static int fuzz_residual(void) {
 			((uint8_t *)(ctx.t.pps.weightScale8x8_v + inter * 4))[j * 8 + i] = sc8[i * 8 + j];
 		}
 		add_idct8x8(&ctx, 0, pix + 32 * 6 + 16);
+		d = fnv(d, pix, sizeof(pix));
 		port_idct8x8(lv8, sc8, qp, res8);
 		for (int y = 0; y < 8; y++) for (int x = 0; x < 8; x++) want[32 * (6 + y) + 16 + x] = (uint8_t)clip8((int16_t)(want[32 * (6 + y) + 16 + x] + res8[y * 8 + x]));
 		if (memcmp(want, pix, sizeof(pix))) { if (bad++ < 5) printf("IDCT8x8 MISMATCH trial %d qp %d inter %d extreme %d\n", trial, qp, inter, extreme); memcpy(want, pix, sizeof(pix)); }
@@ -122,6 +134,7 @@ static int fuzz_residual(void) {
 			static const uint8_t zr[16] = {0, 1, 4, 5, 2, 3, 6, 7, 8, 9, 12, 13, 10, 11, 14, 15};
 			int ok = 1;
 			for (int b = 0; b < 16; b++) if (ctx.c[16 + b] != dcs[zr[b]]) ok = 0;
+			for (int b = 0; b < 16; b++) { int32_t v = ctx.c[16 + b]; d = fnv(d, &v, 4); }
 			if (!ok && bad++ < 5) { printf("LUMA DC MISMATCH trial %d qp %d:", trial, qp); for (int b = 0; b < 16; b++) printf(" %d/%d", ctx.c[16 + b], dcs[zr[b]]); printf("\n"); }
 		}
 		memset(ctx.c, 0, sizeof(ctx.c));
@@ -139,6 +152,8 @@ static int fuzz_residual(void) {
 		{
 			int ok = 1;
 			for (int i = 0; i < 4; i++) if (ctx.c[16 + i] != dcb[i] || ctx.c[20 + i] != dcr[i]) ok = 0;
+			for (int i = 0; i < 8; i++) { int32_t v = ctx.c[16 + i]; d = fnv(d, &v, 4); }
+			put_digest(d);
 			if (!ok && bad++ < 5) { printf("CHROMA DC MISMATCH trial %d:", trial); for (int i = 0; i < 4; i++) printf(" %d/%d %d/%d", ctx.c[16 + i], dcb[i], ctx.c[20 + i], dcr[i]); printf("\n"); }
 		}
 		memset(ctx.c, 0, sizeof(ctx.c));
@@ -204,6 +219,7 @@ static int fuzz_deblock(void) {
 			}
 		}
 		deblock_Y_8bit(&ctx);
+		put_digest(fnv(fnv(2166136261u, y, sizeof(y)), c, sizeof(c)));
 		if (memcmp(wy, y, sizeof(y)) || memcmp(wc, c, sizeof(c))) {
 			if (bad++ < 6) {
 				int py = -1, pc = -1;
@@ -249,10 +265,11 @@ static int dump_kat(void) {
 }
 
 int main(int argc, char **argv) {
+	if (argc > 3 && !strcmp(argv[2], "--digests") && !(digests = fopen(argv[3], "wb"))) { perror(argv[3]); return 2; }
 	if (argc > 1 && !strcmp(argv[1], "fuzz")) return fuzz_inter() != 0;
 	if (argc > 1 && !strcmp(argv[1], "residual")) return fuzz_residual() != 0;
 	if (argc > 1 && !strcmp(argv[1], "deblock")) return fuzz_deblock() != 0;
 	if (argc > 1 && !strcmp(argv[1], "dump")) return dump_kat();
-	fprintf(stderr, "usage: ref_kat fuzz | residual | deblock | dump\n");
+	fprintf(stderr, "usage: ref_kat fuzz | residual | deblock [--digests FILE] | dump\n");
 	return 2;
 }

@@ -1,10 +1,21 @@
 """API behaviour beyond the plain decode loop, compared between the reference and our host code (CPU backend):
 borrowed frames (edge264_get_frame(borrow=1) / edge264_return_frame, reference edge264.c:365-414), flush in the middle
-of a stream (edge264.c:261-270), and the sequence of return codes of edge264_decode_NAL."""
-import ctypes, errno, os
+of a stream (edge264.c:261-270), and the sequence of return codes of edge264_decode_NAL.  What the reference answered
+is recorded in tests/golden/api_reference.json (tests/make_golden.py)."""
+import ctypes, errno, hashlib, json, os
 import pytest
-from conftest import STREAMS, make_stream, have
+from conftest import ROOT, STREAMS, make_stream
 from checkers import load, Edge264Frame, _frame_bytes
+
+
+
+@pytest.fixture(scope="module")
+def gold():
+    return json.load(open(os.path.join(ROOT, "tests", "golden", "api_reference.json")))
+
+
+def digests(frames):
+    return [[f[0], hashlib.md5(f[3]).hexdigest()] for f in frames]
 
 
 def decode_borrowing(data, backend, hold, flush_at=None):
@@ -62,27 +73,24 @@ CASES = [STREAMS[6], STREAMS[8], STREAMS[9]]   # I P B B streams: frames leave o
 
 @pytest.mark.parametrize("name,w,h,args", CASES, ids=[c[0] for c in CASES])
 @pytest.mark.parametrize("hold", [1, 3])
-def test_borrowed_frames_match_reference(workdir, name, w, h, args, hold):
+def test_borrowed_frames_match_reference(workdir, gold, name, w, h, args, hold):
     data = open(make_stream(workdir, name, w, h, args), "rb").read()
     plain, _ = decode_borrowing(data, "port", 0)
     ours, codes = decode_borrowing(data, "port", hold)
     assert [(f[0], f[3]) for f in ours] == [(f[0], f[3]) for f in plain], "holding frames changed the output"
-    if have("ref"):
-        ref, rcodes = decode_borrowing(data, "ref", hold)
-        assert [(f[0], f[3]) for f in ref] == [(f[0], f[3]) for f in ours]
-        assert rcodes == codes, "edge264_decode_NAL return codes differ from the reference's"
+    ref = gold["borrowed"][f"{name}/{hold}"]
+    assert ref["frames"] == digests(ours)
+    assert ref["codes"] == codes, "edge264_decode_NAL return codes differ from the reference's"
 
 
-def test_flush_mid_stream_matches_reference(workdir):
+def test_flush_mid_stream_matches_reference(workdir, gold):
     name, w, h, args = STREAMS[6]
     data = open(make_stream(workdir, name, w, h, args), "rb").read()
-    if not have("ref"):
-        pytest.skip("reference library not built")
     for at in (7, 12):
         ours, codes = decode_borrowing(data, "port", 0, flush_at=at)
-        ref, rcodes = decode_borrowing(data, "ref", 0, flush_at=at)
-        assert rcodes == codes
-        assert [(f[0], f[3]) for f in ref] == [(f[0], f[3]) for f in ours]
+        ref = gold["flush"][str(at)]
+        assert ref["codes"] == codes
+        assert ref["frames"] == digests(ours)
 
 
 UNREF = ctypes.CFUNCTYPE(None, ctypes.c_int, ctypes.c_void_p)
@@ -114,14 +122,12 @@ def decode_with_unref(data, backend):
     return log
 
 
-def test_unref_callback_matches_reference(workdir):
+def test_unref_callback_matches_reference(workdir, gold):
     """n_threads = 0: the reference calls unref_cb(ret, arg) exactly once before edge264_decode_NAL returns, for slices and
     for every other NAL (edge264.c:356-357, edge264_headers.c:497-498)."""
-    if not have("ref"):
-        pytest.skip("reference library not built")
     for name, w, h, args in (STREAMS[2], STREAMS[6]):
         data = open(make_stream(workdir, name, w, h, args), "rb").read()
-        assert decode_with_unref(data, "port") == decode_with_unref(data, "ref")
+        assert json.loads(json.dumps(decode_with_unref(data, "port"))) == gold["unref"][name]
 
 
 def _split_nals(b):
@@ -134,31 +140,29 @@ def _split_nals(b):
     return [b[idx[k]:(idx[k + 1] if k + 1 < len(idx) else len(b))] for k in range(len(idx))]
 
 
-@pytest.mark.parametrize("case", [("-W 3 -H 2 -n 12 -s 90292 --gop IPB --refs 5 --idr 17 --deblock 0 --wp 1", [8]),
-                                  ("-W 3 -H 3 -n 10 -s 31 --gop IP --refs 3 --deblock 0", [5]),
-                                  ("-W 2 -H 3 -n 30 -s 90293 --gop IPB --refs 5 --idr 9 --deblock 0 --wp 2", [24, 34, 44])],
-                         ids=["ipb_one_anchor", "ip_one_picture", "ipb_three_anchors"])
-def test_lost_reference_pictures_follow_the_reference(workdir, case):
+LOST_CASES = [("-W 3 -H 2 -n 12 -s 90292 --gop IPB --refs 5 --idr 17 --deblock 0 --wp 1", [8]),
+              ("-W 3 -H 3 -n 10 -s 31 --gop IP --refs 3 --deblock 0", [5]),
+              ("-W 2 -H 3 -n 30 -s 90293 --gop IPB --refs 5 --idr 9 --deblock 0 --wp 2", [24, 34, 44])]
+
+
+@pytest.mark.parametrize("case", LOST_CASES, ids=["ipb_one_anchor", "ip_one_picture", "ipb_three_anchors"])
+def test_lost_reference_pictures_follow_the_reference(workdir, gold, case):
     """A lost reference picture is a gap in frame_num (8.2.5.2): like the reference (edge264_headers.c:1095-1139) we insert
     non-existing frames, so the number of output frames, their order and their FrameIds must match.  Samples of pictures
     predicted from a non-existing frame are undefined in the reference (never-written buffers) and are not compared,
     except that everything output before the loss must be identical."""
     import subprocess
-    from conftest import ROOT
+    from conftest import md5_frames
     from checkers import decode_bytes
-    if not have("ref"):
-        pytest.skip("reference library not built")
     args, drop = case
     path = os.path.join(workdir, "gap_%d.264" % abs(hash(args)))
     subprocess.run([os.path.join(ROOT, "tools", "gen264"), "-o", path] + args.split(), check=True, stderr=subprocess.DEVNULL)
     nals = _split_nals(open(path, "rb").read())
     data = b"".join(n for k, n in enumerate(nals) if k not in drop)
-    ref, _ = decode_bytes(data, "ref")
+    ref = gold["lost"][args]      # md5_before: the reference's pictures complete and output-ordered before the first loss
     ours, _ = decode_bytes(data, "port")
-    assert [(f[0], f[1], f[2]) for f in ours] == [(f[0], f[1], f[2]) for f in ref]
-    intact, _ = decode_bytes(b"".join(nals[:min(drop)]), "ref")
-    n_before = max(0, len(intact) - 3)     # pictures complete and output-ordered before the first loss
-    assert [f[3] for f in ours[:n_before]] == [f[3] for f in ref[:n_before]]
+    assert [[f[0], f[1], f[2]] for f in ours] == ref["frames"]
+    assert md5_frames(ours[:len(ref["md5_before"])]) == ref["md5_before"]
 
 
 ALLOC = ctypes.CFUNCTYPE(None, ctypes.POINTER(ctypes.c_void_p), ctypes.c_uint, ctypes.POINTER(ctypes.c_void_p), ctypes.c_uint, ctypes.c_int, ctypes.c_void_p)
@@ -209,27 +213,20 @@ def decode_with_allocator(data, backend):
     return out, allocs, len(frees), len(live)
 
 
-def test_application_allocator_is_used_and_balanced(workdir):
+def test_application_allocator_is_used_and_balanced(workdir, gold):
     name, w, h, args = STREAMS[6]
     data = open(make_stream(workdir, name, w, h, args), "rb").read()
     frames, allocs, n_free, leaked = decode_with_allocator(data, "port")
     plain, _ = decode_borrowing(data, "port", 0)
     assert [(f[0], f[1]) for f in frames] == [(f[0], f[3]) for f in plain]
     assert allocs and n_free == len(allocs) and leaked == 0, "every buffer obtained from alloc_cb must go back through free_cb"
-    if have("ref"):
-        rframes, rallocs, rfree, rleak = decode_with_allocator(data, "ref")
-        assert [(f[0], f[1]) for f in rframes] == [(f[0], f[1]) for f in frames]
-        assert set(rallocs) == set(allocs), "buffer sizes requested from the application differ from the reference's"
+    ref = gold["allocator"]
+    assert ref["frames"] == [[f[0], hashlib.md5(f[1]).hexdigest()] for f in frames]
+    assert ref["allocs"] == [list(a) for a in sorted(set(allocs))], "buffer sizes requested from the application differ from the reference's"
 
 
-def test_sequence_changes_follow_the_reference(workdir):
-    """Several coded video sequences in one stream: new sizes and crops (the reference clears its decoder), and a change of
-    max_num_ref_frames alone (it does not: FrameId numbering and parameter sets continue, edge264_headers.c:2016-2024)."""
+def sequence_changes_stream(workdir):
     import subprocess
-    from conftest import ROOT, md5_frames
-    from checkers import decode_bytes
-    if not have("ref"):
-        pytest.skip("reference library not built")
     parts = []
     for k, a in enumerate(["-W 9 -H 7 -n 7 -s 13 --gop IPB --deblock 0", "-W 6 -H 5 -n 6 -s 14 --gop IP --refs 3 --deblock 0 --cavlc",
                            "-W 9 -H 7 -n 5 -s 15 --gop IPB --refs 4 --deblock 0", "-W 9 -H 7 -n 7 -s 13 --gop IPB --deblock 0",
@@ -237,8 +234,15 @@ def test_sequence_changes_follow_the_reference(workdir):
         p = os.path.join(workdir, "seq_%d.264" % k)
         subprocess.run([os.path.join(ROOT, "tools", "gen264"), "-o", p] + a.split(), check=True, stderr=subprocess.DEVNULL)
         parts.append(open(p, "rb").read())
-    data = b"".join(parts)
-    ref, rc = decode_bytes(data, "ref")
-    ours, oc = decode_bytes(data, "port")
-    assert [(f[0], f[1], f[2]) for f in ours] == [(f[0], f[1], f[2]) for f in ref]
-    assert md5_frames(ours) == md5_frames(ref) and oc == rc
+    return b"".join(parts)
+
+
+def test_sequence_changes_follow_the_reference(workdir, gold):
+    """Several coded video sequences in one stream: new sizes and crops (the reference clears its decoder), and a change of
+    max_num_ref_frames alone (it does not: FrameId numbering and parameter sets continue, edge264_headers.c:2016-2024)."""
+    from conftest import md5_frames
+    from checkers import decode_bytes
+    ref = gold["sequence"]
+    ours, oc = decode_bytes(sequence_changes_stream(workdir), "port")
+    assert [[f[0], f[1], f[2]] for f in ours] == ref["frames"]
+    assert md5_frames(ours) == ref["md5"] and oc == ref["codes"]

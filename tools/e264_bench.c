@@ -13,7 +13,7 @@
 #include "edge264.h"
 
 typedef struct Job {
-	const uint8_t *buf; size_t size;
+	int stream; const uint8_t *buf; size_t size;
 	long frames; uint64_t sum; int last_ret;
 	Edge264Decoder *dec; int keep;
 } Job;
@@ -34,6 +34,22 @@ static uint64_t frame_sum(const Edge264Frame *f) {
 	return s;
 }
 
+/* frames copied out during e264bench_run (bench.py --dump-outputs), set by e264bench_capture */
+static struct { int n; const int *stream; const long *index; uint8_t **dst; size_t cap; int *info; } capture;
+
+static void capture_frame(const Job *j, long index, const Edge264Frame *f) {
+	for (int k = 0; k < capture.n; k++) {
+		if (capture.stream[k] != j->stream || capture.index[k] != index) continue;
+		uint8_t *d = capture.dst[k], *e = d + capture.cap;
+		for (int pl = 0; pl < 3; pl++) {
+			int w = pl ? f->width_C : f->width_Y, h = pl ? f->height_C : f->height_Y, st = pl ? f->stride_C : f->stride_Y;
+			for (int y = 0; y < h && d + w <= e; y++, d += w) memcpy(d, f->samples[pl] + (size_t)y * st, (size_t)w);
+		}
+		int *info = capture.info + 5 * k;
+		info[0] = f->FrameId; info[1] = f->width_Y; info[2] = f->height_Y; info[3] = f->width_C; info[4] = f->height_C;
+	}
+}
+
 static void decode_stream(Job *j) {
 	const uint8_t *buf = j->buf, *end = buf + j->size;
 	const uint8_t *nal = buf + 3 + (buf[2] == 0);
@@ -48,7 +64,11 @@ static void decode_stream(Job *j) {
 		long before = frames;
 		res = edge264_decode_NAL(dec, nal, sc, NULL, NULL);
 		if (nal >= end) drained = 1;
-		while (!edge264_get_frame(dec, &f, 0)) { sum = sum * 31 + frame_sum(&f); frames++; }
+		while (!edge264_get_frame(dec, &f, 0)) {
+			sum = sum * 31 + frame_sum(&f);
+			if (capture.n) capture_frame(j, frames, &f);
+			frames++;
+		}
 		if (res == ENOBUFS) { if (frames == before) break; continue; }
 		if (res == ENOTSUP || res == EBADMSG) res = 0;
 		nal = sc + 3 < end ? sc + 3 : end;
@@ -76,7 +96,7 @@ static void *worker(void *arg) {
 double e264bench_run(const uint8_t **bufs, const size_t *sizes, int n_streams, int n_threads, int keep,
                      long *frames, uint64_t *sums, void **decoders) {
 	Job *jobs = (Job *)calloc((size_t)n_streams, sizeof(Job));
-	for (int i = 0; i < n_streams; i++) { jobs[i].buf = bufs[i]; jobs[i].size = sizes[i]; jobs[i].keep = keep; }
+	for (int i = 0; i < n_streams; i++) { jobs[i].stream = i; jobs[i].buf = bufs[i]; jobs[i].size = sizes[i]; jobs[i].keep = keep; }
 	if (n_threads > n_streams) n_threads = n_streams;
 	if (n_threads < 1) n_threads = 1;
 	pthread_barrier_t bar; pthread_barrier_init(&bar, NULL, (unsigned)n_threads + 1);
@@ -91,5 +111,11 @@ double e264bench_run(const uint8_t **bufs, const size_t *sizes, int n_streams, i
 	for (int i = 0; i < n_streams; i++) { if (frames) frames[i] = jobs[i].frames; if (sums) sums[i] = jobs[i].sum; if (decoders) decoders[i] = jobs[i].dec; }
 	free(th); free(jobs); pthread_barrier_destroy(&bar);
 	return (t1.tv_sec - t0.tv_sec) + 1e-9 * (t1.tv_nsec - t0.tv_nsec);
+}
+/* Output frames to copy during the following e264bench_run calls: frame index[k] (in output order) of stream stream[k]
+ * goes to dst[k] (at most cap bytes: the cropped Y, Cb and Cr planes one after the other), its FrameId, width_Y,
+ * height_Y, width_C and height_C to info[5k..5k+4].  n = 0 ends the capture. */
+void e264bench_capture(int n, const int *stream, const long *index, uint8_t **dst, size_t cap, int *info) {
+	capture.stream = stream; capture.index = index; capture.dst = dst; capture.cap = cap; capture.info = info; capture.n = n;
 }
 void e264bench_free(void **decoders, int n) { for (int i = 0; i < n; i++) { Edge264Decoder *d = (Edge264Decoder *)decoders[i]; edge264_free(&d); decoders[i] = NULL; } }
