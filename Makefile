@@ -17,11 +17,12 @@ $(CSRC)/slice_dec.o: $(CSRC)/slice_dec.c $(wildcard $(CSRC)/*.h)
 $(LIB): $(CSRC)/recon.o $(CSRC)/decoder.o $(CSRC)/slice_dec.o
 	$(NVCC) -shared -o $@ $^ -cudart shared
 # experiment builds of the runtime with other block geometries of the inter kernel (tools/gpu_variants.sh; not part of `all`)
-VARIANTS := w4 w8 timing iw4 iw8
+VARIANTS := w4 w8 timing itiming iw4 iw8
 variants: $(foreach v,$(VARIANTS),edge264_b200/variants/$(v)/libedge264_b200.so)
 edge264_b200/variants/w8/libedge264_b200.so: VFLAGS := -DINTER_WARPS=8
 edge264_b200/variants/w4/libedge264_b200.so: VFLAGS := -DINTER_WARPS=4
 edge264_b200/variants/timing/libedge264_b200.so: VFLAGS := -DE264_ROWS_TIMING
+edge264_b200/variants/itiming/libedge264_b200.so: VFLAGS := -DE264_INTER_TIMING
 edge264_b200/variants/iw4/libedge264_b200.so: VFLAGS := -DINTRA_WARPS=4
 edge264_b200/variants/iw8/libedge264_b200.so: VFLAGS := -DINTRA_WARPS=8
 edge264_b200/variants/%/libedge264_b200.so: $(CSRC)/recon.cu $(wildcard $(CSRC)/*.cuh) $(wildcard $(CSRC)/*.h) $(CSRC)/decoder.o $(CSRC)/slice_dec.o

@@ -33,30 +33,35 @@ struct __align__(16) E264DbkMb {
 
 __device__ __forceinline__ int dbk_iabs(int v) { return v < 0 ? -v : v; }
 
-__device__ int dbk_bs_pair(const E264MbRec *p, int bp, const E264MbRec *q, int bq, bool mb_edge) {
-	if (p->kind != MBK_INTER || q->kind != MBK_INTER) return mb_edge ? 4 : 3;
-	if (((p->coded >> bp) & 1) || ((q->coded >> bq) & 1)) return 2;
-	int p0 = p->ref_idx[0][bp >> 2] < 0 ? -1 : p->ref_pic[0][bp >> 2], p1 = p->ref_idx[1][bp >> 2] < 0 ? -1 : p->ref_pic[1][bp >> 2];
-	int q0 = q->ref_idx[0][bq >> 2] < 0 ? -1 : q->ref_pic[0][bq >> 2], q1 = q->ref_idx[1][bq >> 2] < 0 ? -1 : q->ref_pic[1][bq >> 2];
-	if (!((p0 == q0 && p1 == q1) || (p0 == q1 && p1 == q0))) return 1;
+/* bS of one edge segment between 4x4 block bp of p and bq of q (8.7.2.1), every condition evaluated and the answer
+ * selected: the lanes of a warp reach different answers, and early returns made the warp run them one after another */
+__device__ __forceinline__ int dbk_bs_pair(const E264MbRec *p, int bp, const E264MbRec *q, int bq, bool mb_edge) {
+	const bool intra = p->kind != MBK_INTER || q->kind != MBK_INTER;
+	const bool coef = ((p->coded >> bp) & 1) || ((q->coded >> bq) & 1);
+	const int p0 = p->ref_idx[0][bp >> 2] < 0 ? -1 : p->ref_pic[0][bp >> 2], p1 = p->ref_idx[1][bp >> 2] < 0 ? -1 : p->ref_pic[1][bp >> 2];
+	const int q0 = q->ref_idx[0][bq >> 2] < 0 ? -1 : q->ref_pic[0][bq >> 2], q1 = q->ref_idx[1][bq >> 2] < 0 ? -1 : q->ref_pic[1][bq >> 2];
+	const bool same = (p0 == q0 && p1 == q1) || (p0 == q1 && p1 == q0);
 #define FAR(lp, lq) (dbk_iabs(p->mv[lp][bp][0] - q->mv[lq][bq][0]) >= 4 || dbk_iabs(p->mv[lp][bp][1] - q->mv[lq][bq][1]) >= 4)
-	if (p0 >= 0 && p1 >= 0) {
-		if (p0 != p1) return (p0 == q0) ? (FAR(0, 0) || FAR(1, 1)) : (FAR(0, 1) || FAR(1, 0));
-		return (FAR(0, 0) || FAR(1, 1)) && (FAR(0, 1) || FAR(1, 0));
-	}
-	int lp = p0 >= 0 ? 0 : 1, lq = q0 >= 0 ? 0 : 1;
-	return FAR(lp, lq);
+	const bool f00 = FAR(0, 0), f11 = FAR(1, 1), f01 = FAR(0, 1), f10 = FAR(1, 0);
 #undef FAR
+	const bool bi = p0 >= 0 && p1 >= 0;
+	const bool two = p0 != p1 ? (p0 == q0 ? f00 || f11 : f01 || f10) : (f00 || f11) && (f01 || f10);
+	const bool one = p0 >= 0 ? (q0 >= 0 ? f00 : f01) : (q0 >= 0 ? f10 : f11);
+	const int mvbs = (bi ? two : one) ? 1 : 0;
+	return intra ? (mb_edge ? 4 : 3) : coef ? 2 : !same ? 1 : mvbs;
 }
 
 /* digest of one macroblock by one warp: 32 boundary strengths (one lane per edge segment), thresholds of the nine plane x
- * edge-kind combinations.  recs: 3 x 12 uint4 of shared memory for the warp, dg: 64 bytes of shared memory. */
-__device__ __forceinline__ void dbk_digest_mb(const PicJob &J, uint4 (*recs)[12], E264DbkMb *dg, int mb, int lane) {
+ * edge-kind combinations.  recs: 3 x 12 uint4 of shared memory for the warp, dg: 64 bytes of shared memory.  cur, left,
+ * top: the records of the macroblock and its neighbours where the caller already holds them in shared memory, else
+ * nullptr (they are then fetched into recs). */
+__device__ __forceinline__ void dbk_digest_mb(const PicJob &J, uint4 (*recs)[12], E264DbkMb *dg, int mb, int lane,
+                                              const E264MbRec *cur = nullptr, const E264MbRec *left = nullptr, const E264MbRec *top = nullptr) {
 	const int W = J.w_mbs, mbx = mb % W, mby = mb / W;
-	const E264MbRec *q = (const E264MbRec *)recs[0], *pL = (const E264MbRec *)recs[1], *pT = (const E264MbRec *)recs[2];
-	if (lane < 12) recs[0][lane] = __ldg((const uint4 *)(J.recs + mb) + lane);
-	else if (lane < 24) { if (mbx > 0) recs[1][lane - 12] = __ldg((const uint4 *)(J.recs + mb - 1) + lane - 12); }
-	if (lane < 12 && mby > 0) recs[2][lane] = __ldg((const uint4 *)(J.recs + mb - W) + lane);
+	const E264MbRec *q = cur ? cur : (const E264MbRec *)recs[0], *pL = left ? left : (const E264MbRec *)recs[1], *pT = top ? top : (const E264MbRec *)recs[2];
+	if (lane < 12) { if (!cur) recs[0][lane] = __ldg((const uint4 *)(J.recs + mb) + lane); }
+	else if (lane < 24) { if (!left && mbx > 0) recs[1][lane - 12] = __ldg((const uint4 *)(J.recs + mb - 1) + lane - 12); }
+	if (lane < 12 && !top && mby > 0) recs[2][lane] = __ldg((const uint4 *)(J.recs + mb - W) + lane);
 	__syncwarp();
 	const int qflags = q->flags;
 	const bool on_mb = qflags & MBF_DEBLOCK, fl = qflags & MBF_EDGE_L, ft = qflags & MBF_EDGE_T, t8 = qflags & MBF_T8x8;
@@ -66,7 +71,8 @@ __device__ __forceinline__ void dbk_digest_mb(const PicJob &J, uint4 (*recs)[12]
 		const E264MbRec *p = q;
 		bool on = on_mb && !(t8 && (e & 1));
 		if (e == 0) { on = on && (dir ? ft : fl); p = dir ? pT : pL; }
-		if (on) {
+		if (q->kind != MBK_INTER) bs = on ? (e == 0 ? 4 : 3) : 0;     /* intra macroblock: no per-lane work */
+		else if (on) {
 			const int qx = dir ? k : e, qy = dir ? e : k;
 			const int px_ = dir ? k : (e ? e - 1 : 3), py_ = dir ? (e ? e - 1 : 3) : k;
 			bs = dbk_bs_pair(p, blk_z(px_, py_), q, blk_z(qx, qy), e == 0);

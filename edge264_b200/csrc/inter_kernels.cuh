@@ -6,8 +6,9 @@
  * windows of neighbouring blocks overlap in L1/L2) and interpolates 4x4 + 2x2 + 2x2 samples with the register arithmetic of
  * mc_math.cuh (dp4a tap sums).  Items are binned by interpolation class so that a warp runs ONE class body on 32 items
  * (reference edge264_inter.c:416-1251: per-partition SIMD interpolation + five weighting schemes).
- * The macroblock's coefficient run (16..816 bytes) arrives by cp.async.bulk on an mbarrier one macroblock ahead and is
- * inverse-transformed in shared memory (residual_stage), so the residual never travels through global memory.
+ * The macroblock's coefficient run (16..816 bytes) arrives by cp.async.bulk on an mbarrier one macroblock ahead; each 4x4
+ * block is inverse-transformed by the lane that also weights and stores it, so the residual stays in registers (only the
+ * 8x8 transform passes through shared memory).
  * History: round 1's kernel (rectangles regrouped on the device, windows by cp.async.bulk.tensor into shared memory, one
  * output sample per lane and loop iteration) needed ~3600 warp instructions per macroblock and 77 us per 1080p picture;
  * this one 1630 and 39 us, and 35 k pictures/s with 32 streams in flight since its blocks are 16 warps in lock-step phases
@@ -78,12 +79,23 @@ __device__ __forceinline__ uint32_t wp_word(uint32_t a, uint32_t b, int wa, int 
 	}
 	return r;
 }
-/* prediction + residual of four packed samples; res points at four int16 (8-byte aligned) */
-__device__ __forceinline__ uint32_t add_res4(uint32_t p, const int16_t *res) {
-	const uint2 rr = *(const uint2 *)res;
-	const int r0 = (short)(rr.x & 0xffff), r1 = (short)(rr.x >> 16), r2 = (short)(rr.y & 0xffff), r3 = (short)(rr.y >> 16);
-	return mc_pack4(clip255((short)((int)(p & 255) + r0)), clip255((short)((int)((p >> 8) & 255) + r1)),
-	                clip255((short)((int)((p >> 16) & 255) + r2)), clip255((short)((int)(p >> 24) + r3)));
+/* prediction + residual of four packed samples; res: four int16 residuals */
+__device__ __forceinline__ uint32_t add_res4(uint32_t p, const int res[4]) {
+	return mc_pack4(clip255((short)((int)(p & 255) + res[0])), clip255((short)((int)((p >> 8) & 255) + res[1])),
+	                clip255((short)((int)((p >> 16) & 255) + res[2])), clip255((short)((int)(p >> 24) + res[3])));
+}
+/* the four prediction rows of one list for the lane's 4x4 block of samples (see phase 3): a luma lane's block as it was
+ * stored; chroma lane 16 + 4 pl + i joins the 2x2 predictions of plane pl of luma blocks 4i..4i+3 (a 2x2 word holds row 0
+ * in its low, row 1 in its high half) */
+__device__ __forceinline__ void inter_pred_words(const uint32_t (*pred)[8], int lane, uint32_t w[4]) {
+	if (lane < 16) {
+		const uint4 a = *(const uint4 *)pred[lane];
+		w[0] = a.x; w[1] = a.y; w[2] = a.z; w[3] = a.w;
+	} else {
+		const int j = lane - 16, z = (j & 3) * 4, e = 4 + (j >> 2);
+		const uint32_t a = pred[z][e], b = pred[z + 1][e], c = pred[z + 2][e], d = pred[z + 3][e];
+		w[0] = __byte_perm(a, b, 0x5410); w[1] = __byte_perm(a, b, 0x7632); w[2] = __byte_perm(c, d, 0x5410); w[3] = __byte_perm(c, d, 0x7632);
+	}
 }
 
 /* ---- the kernel ----
@@ -114,7 +126,7 @@ struct __align__(16) InterSmem {
 	uint16_t queue[6][INTER_CHUNK * 32];           /* item = macroblock << 5 | list << 4 | luma4x4BlkIdx */
 	int qn[6];
 	WarpSmem ws[INTER_WARPS];
-	uint4 drecs[INTER_WARPS][3][12];               /* deblocking digests: records of the current, left and top macroblock per warp */
+	uint4 drecs[INTER_WARPS][3][12];               /* deblocking digests: records of neighbours outside the chunk (left, top) per warp */
 	E264DbkMb ddg[INTER_WARPS];
 	int16_t coef[INTER_WARPS][2][RES_COEF_MAX];
 	unsigned long long bars[INTER_WARPS][2];
@@ -172,11 +184,13 @@ __global__ void __launch_bounds__(INTER_WARPS * 32, MINB) e264_inter4_kernel(Pic
 		asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
 		asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
 	}
-	unsigned parity[2] = {0, 0};
+	unsigned parity = 0;      /* bit b: phase parity of bars[w][b] (a bit mask, not an array: b is not a constant) */
 	const int nchunks = (nmb + INTER_CHUNK - 1) / INTER_CHUNK;
+	IT_DECL
 	for (int chunk = blockIdx.x; chunk < nchunks; chunk += gridDim.x) {
 		const int mb0 = chunk * INTER_CHUNK, cnt = min(INTER_CHUNK, nmb - mb0);
 		__syncthreads();                               /* the previous chunk's predictions and records are no longer read */
+		IT_MARK(4)
 		/* ---- 1. records, queues ---- */
 		for (int i = tid; i < cnt * 12; i += INTER_WARPS * 32) sm.rec4[i / 12][i % 12] = __ldg((const uint4 *)(J.recs + mb0) + i);
 		if (tid < 6) sm.qn[tid] = 0;
@@ -209,6 +223,7 @@ __global__ void __launch_bounds__(INTER_WARPS * 32, MINB) e264_inter4_kernel(Pic
 			if (cls >= 0) sm.queue[cls][base + __popc(peers & ((1u << lane) - 1))] = (uint16_t)item;
 		}
 		__syncthreads();
+		IT_MARK(0)
 		/* ---- 2. one class at a time, 32 items per warp pass: the groups of all classes form one list ---- */
 		{
 			int total = 0;
@@ -224,70 +239,104 @@ __global__ void __launch_bounds__(INTER_WARPS * 32, MINB) e264_inter4_kernel(Pic
 			}
 		}
 		__syncthreads();
+		IT_MARK(1)
 		/* ---- 3. a warp per macroblock: inverse transform, weighting, residual, store ---- */
 		int b = 0;
 		bool failed = false;
 #pragma unroll 1
 		for (int m = w; m < cnt; m += INTER_WARPS, b ^= 1) {
 			const int what2 = coef_issue(m + INTER_WARPS, b ^ 1);
-			/* the macroblock's deblocking digest (every macroblock, intra ones too): record-only work whose loads of the
-			 * neighbour records are in flight together with the coefficient run requested above */
-			if (J.dbk != nullptr) dbk_digest_mb(J, sm.drecs[w], &sm.ddg[w], mb0 + m, lane);
+			/* the macroblock's deblocking digest (every macroblock, intra ones too): record-only work whose load of the
+			 * record above is in flight together with the coefficient run requested above; the current and left records
+			 * (and the one above in pictures narrower than a chunk) are the chunk's */
+			if (J.dbk != nullptr)
+				dbk_digest_mb(J, sm.drecs[w], &sm.ddg[w], mb0 + m, lane, (const E264MbRec *)sm.rec4[m], m > 0 ? (const E264MbRec *)sm.rec4[m - 1] : nullptr,
+				              m >= J.w_mbs ? (const E264MbRec *)sm.rec4[m - J.w_mbs] : nullptr);
+			IT_MARK(2)
 			if (what) {
 				const int mb = mb0 + m, mbx = mb % J.w_mbs, mby = mb / J.w_mbs;
 				const E264MbRec *r = (const E264MbRec *)sm.rec4[m];
 				const E264SliceRec *sr = J.slices + r->slice_idx;
+				const unsigned coded = r->coded;
+				const bool t8 = r->flags & MBF_T8x8;
+				const int16_t *cf = sm.coef[w][b];
 				if (what == 2) {
-					if (!mbar_wait(&sm.bars[w][b], parity[b])) { if (lane == 0) atomicExch(J.err, 4u); failed = true; }
-					parity[b] ^= 1;
-					if (!failed) residual_stage(ws, r, sr, sm.coef[w][b], lane);
+					if (!mbar_wait(&sm.bars[w][b], (parity >> b) & 1)) { if (lane == 0) atomicExch(J.err, 4u); failed = true; }
+					parity ^= 1u << b;
+					if (coded & CODED_Y_DC) cf += 16;     /* Intra16x16 only: not in an inter macroblock's run */
+					if (!failed && t8 && (coded & 0x1111)) residual_luma8x8(ws, r, sr, cf, lane);
 				}
-				if (lane < 16 && !failed) {
-					const int z = lane, bx = blk_x(z), by = blk_y(z), i8 = z >> 2;
+				IT_MARK(3)
+				/* a lane per 4x4 block of samples: lanes 0-15 luma block z = lane, lane 16 + 4 pl + i chroma block i of plane
+				 * pl (the 2x2 predictions of luma blocks 4i..4i+3); prediction, weighting, residual in registers, store */
+				if (lane < 24 && !failed) {
+					const bool luma = lane < 16;
+					const int j = lane - 16, pl = (j >> 2) & 1, i8 = luma ? lane >> 2 : j & 3;
 					const int r0 = r->ref_idx[0][i8], r1 = r->ref_idx[1][i8];
-					uint32_t py[4] = {0, 0, 0, 0}, pcb = 0, pcr = 0, qy[4] = {0, 0, 0, 0}, qcb = 0, qcr = 0;
-					if (r0 >= 0) { const uint4 a = *(const uint4 *)sm.pred[m][0][z]; const uint2 c2 = *(const uint2 *)(sm.pred[m][0][z] + 4); py[0] = a.x; py[1] = a.y; py[2] = a.z; py[3] = a.w; pcb = c2.x; pcr = c2.y; }
-					if (r1 >= 0) { const uint4 a = *(const uint4 *)sm.pred[m][1][z]; const uint2 c2 = *(const uint2 *)(sm.pred[m][1][z] + 4); qy[0] = a.x; qy[1] = a.y; qy[2] = a.z; qy[3] = a.w; qcb = c2.x; qcr = c2.y; }
+					uint32_t p[4] = {0, 0, 0, 0}, q[4] = {0, 0, 0, 0};
+					if (r0 >= 0) inter_pred_words(sm.pred[m][0], lane, p);
+					if (r1 >= 0) inter_pred_words(sm.pred[m][1], lane, q);
 					const int wpm = sr->wp_mode;
 					const bool bi = r0 >= 0 && r1 >= 0;
 					if (!bi && r0 < 0) {
 #pragma unroll
-						for (int k = 0; k < 4; k++) py[k] = qy[k];
-						pcb = qcb; pcr = qcr;
+						for (int k = 0; k < 4; k++) p[k] = q[k];
 					}
 					if (bi && wpm == WP_DEFAULT) {
 #pragma unroll
-						for (int k = 0; k < 4; k++) py[k] = mc_avg4(py[k], qy[k]);
-						pcb = mc_avg4(pcb, qcb); pcr = mc_avg4(pcr, qcr);
+						for (int k = 0; k < 4; k++) p[k] = mc_avg4(p[k], q[k]);
 					} else if ((bi && wpm != WP_DEFAULT) || (wpm == WP_EXPLICIT && (r0 >= 0 || r1 >= 0))) {
-						/* one weighting body for every scheme: parameters per plane, then six words */
-						int wa[3], wb[3], o[3], sh[3], rnd[3];
+						/* one weighting body for every scheme, with the parameters of the lane's plane */
+						const int c = luma ? 0 : 1 + pl, lw = c ? sr->chroma_log2_wd : sr->luma_log2_wd;
 						const int ll = r0 >= 0 ? 0 : 1, ri = (ll ? r1 : r0) & 15;
+						int wa, wb, o, sh, rnd;
+						if (bi && wpm == WP_EXPLICIT) { wa = sr->wp_w[0][r0 & 15][c]; wb = sr->wp_w[1][r1 & 15][c]; o = (sr->wp_o[0][r0 & 15][c] + sr->wp_o[1][r1 & 15][c] + 1) >> 1; sh = lw + 1; rnd = 1 << lw; }
+						else if (bi) { wb = sr->implicit_w1[r0 & 15][r1 & 15]; wa = 64 - wb; o = 0; sh = 6; rnd = 32; }
+						else { wa = sr->wp_w[ll][ri][c]; wb = 0; o = sr->wp_o[ll][ri][c]; sh = lw; rnd = lw >= 1 ? 1 << (lw - 1) : 0; }
 #pragma unroll
-						for (int c = 0; c < 3; c++) {
-							const int lw = c ? sr->chroma_log2_wd : sr->luma_log2_wd;
-							if (bi && wpm == WP_EXPLICIT) { wa[c] = sr->wp_w[0][r0 & 15][c]; wb[c] = sr->wp_w[1][r1 & 15][c]; o[c] = (sr->wp_o[0][r0 & 15][c] + sr->wp_o[1][r1 & 15][c] + 1) >> 1; sh[c] = lw + 1; rnd[c] = 1 << lw; }
-							else if (bi) { wb[c] = sr->implicit_w1[r0 & 15][r1 & 15]; wa[c] = 64 - wb[c]; o[c] = 0; sh[c] = 6; rnd[c] = 32; }
-							else { wa[c] = sr->wp_w[ll][ri][c]; wb[c] = 0; o[c] = sr->wp_o[ll][ri][c]; sh[c] = lw; rnd[c] = lw >= 1 ? 1 << (lw - 1) : 0; }
-						}
-#pragma unroll
-						for (int k = 0; k < 4; k++) py[k] = wp_word(py[k], qy[k], wa[0], wb[0], rnd[0], sh[0], o[0]);
-						pcb = wp_word(pcb, qcb, wa[1], wb[1], rnd[1], sh[1], o[1]); pcr = wp_word(pcr, qcr, wa[2], wb[2], rnd[2], sh[2], o[2]);
+						for (int k = 0; k < 4; k++) p[k] = wp_word(p[k], q[k], wa, wb, rnd, sh, o);
 					}
 					if (what == 2) {
+						int res[16];
+						bool act = false;
+						if (luma && t8) {     /* the 8x8 transform's residual, written above for coded 8x8 blocks only */
+							act = (coded >> lane) & 1;
+							if (act) {
+								const int16_t *rs = ws->res + blk_y(lane) * 64 + blk_x(lane) * 4;
 #pragma unroll
-						for (int k = 0; k < 4; k++) py[k] = add_res4(py[k], ws->res + (by * 4 + k) * 16 + bx * 4);
-						const int16_t *rc = ws->res + 256 + (by * 2) * 8 + bx * 2;
-						const uint32_t a = *(const uint32_t *)rc, bb = *(const uint32_t *)(rc + 8), c2 = *(const uint32_t *)(rc + 64), d = *(const uint32_t *)(rc + 72);
-						pcb = mc_pack4(clip255((short)((int)(pcb & 255) + (short)(a & 0xffff))), clip255((short)((int)((pcb >> 8) & 255) + (short)(a >> 16))),
-						               clip255((short)((int)((pcb >> 16) & 255) + (short)(bb & 0xffff))), clip255((short)((int)(pcb >> 24) + (short)(bb >> 16))));
-						pcr = mc_pack4(clip255((short)((int)(pcr & 255) + (short)(c2 & 0xffff))), clip255((short)((int)((pcr >> 8) & 255) + (short)(c2 >> 16))),
-						               clip255((short)((int)((pcr >> 16) & 255) + (short)(d & 0xffff))), clip255((short)((int)(pcr >> 24) + (short)(d >> 16))));
+								for (int k = 0; k < 4; k++) {
+									const uint2 v = *(const uint2 *)(rs + k * 16);
+									res[4 * k] = (short)(v.x & 0xffff); res[4 * k + 1] = (short)(v.x >> 16); res[4 * k + 2] = (short)(v.y & 0xffff); res[4 * k + 3] = (short)(v.y >> 16);
+								}
+							}
+						} else {
+							const int16_t *cfc = cf + (t8 ? 64 * __popc(coded & 0x1111) : 16 * __popc(coded & 0xffff));   /* chroma DC, then AC */
+							const bool any_cdc = (coded & (CODED_CB_DC | CODED_CR_DC)) != 0;
+							bool on;
+							const int16_t *src; const uint8_t *scal; int qp, dc = 0;
+							if (luma) {
+								on = (coded >> lane) & 1; act = on;
+								src = cf + __popc(coded & ((1u << lane) - 1)) * 16; scal = sr->scaling4x4[3]; qp = r->qp[0];
+							} else {
+								on = (coded >> lane) & 1; act = on || any_cdc;
+								if (any_cdc) dc = chroma_dc(cfc, r, sr, 1, pl, j & 3);
+								src = cfc + (any_cdc ? 8 : 0) + __popc((coded >> 16) & ((1u << j) - 1) & 0xff) * 16; scal = sr->scaling4x4[4 + pl]; qp = r->qp[1 + pl];
+							}
+							if (act) idct4x4_core(src, on, scal, qp, !luma, dc, res);
+						}
+						IT_MARK(3)
+						if (act) {
+#pragma unroll
+							for (int k = 0; k < 4; k++) p[k] = add_res4(p[k], res + 4 * k);
+						}
 					}
+					if (luma) {
 #pragma unroll
-					for (int k = 0; k < 4; k++) *(uint32_t *)&YT(bx * 4, by * 4 + k) = py[k];
-					*(uint16_t *)&CT(0, bx * 2, by * 2) = (uint16_t)pcb; *(uint16_t *)&CT(0, bx * 2, by * 2 + 1) = (uint16_t)(pcb >> 16);
-					*(uint16_t *)&CT(1, bx * 2, by * 2) = (uint16_t)pcr; *(uint16_t *)&CT(1, bx * 2, by * 2 + 1) = (uint16_t)(pcr >> 16);
+						for (int k = 0; k < 4; k++) *(uint32_t *)&YT(blk_x(lane) * 4, blk_y(lane) * 4 + k) = p[k];
+					} else {
+#pragma unroll
+						for (int k = 0; k < 4; k++) *(uint32_t *)&CT(pl, (j & 1) * 4, (j & 2) * 2 + k) = p[k];
+					}
 				}
 				__syncwarp();
 				if (!failed) {
@@ -296,7 +345,9 @@ __global__ void __launch_bounds__(INTER_WARPS * 32, MINB) e264_inter4_kernel(Pic
 				}
 				__syncwarp();
 			}
+			IT_MARK(4)
 			what = what2;
 		}
 	}
+	IT_FLUSH
 }

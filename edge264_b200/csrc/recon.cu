@@ -526,6 +526,18 @@ extern "C" int e264b_replay(E264bDevice **cs, int n, int reps, int threads, E264
 			fprintf(stderr, "\n");
 		}
 	}
+#ifdef E264_INTER_TIMING
+	if (diag) {     /* -DE264_INTER_TIMING builds: cycles per part of a chunk in the inter kernel, all warps summed */
+		unsigned long long ph[16]; cudaMemcpyFromSymbol(ph, g_diag_phase, sizeof ph);
+		unsigned long long tt = 0; for (int k = 0; k < 5; k++) tt += ph[k];
+		const double pics = (double)reps * (double)npic * n;
+		const char *in[5] = {"records+binning", "interpolation", "digest", "residual", "combine+store"};
+		fprintf(stderr, "inter kernel, all warps, %.0f pictures: %.3f Mcycles per picture:", pics, tt / pics * 1e-6);
+		for (int k = 0; k < 5; k++) fprintf(stderr, " %s %.3f (%.1f%%)", in[k], ph[k] / pics * 1e-6, 100.0 * ph[k] / (double)(tt ? tt : 1));
+		fprintf(stderr, "\n");
+	}
+#endif
+#ifdef E264_ROWS_TIMING
 	if (diag) {     /* -DE264_ROWS_TIMING builds: cycles per part of a macroblock step in the intra-picture kernel, all warps summed */
 		unsigned long long ph[16]; cudaMemcpyFromSymbol(ph, g_diag_phase, sizeof ph);
 		unsigned long long tt = 0, tp = 0; for (int k = 0; k < 8; k++) { tt += ph[k]; tp += ph[8 + k]; }
@@ -536,6 +548,7 @@ extern "C" int e264b_replay(E264bDevice **cs, int n, int reps, int threads, E264
 			fprintf(stderr, "rows kernel, prediction warps:"); for (int k = 0; k < 7; k++) fprintf(stderr, " %s %.1f%%", pn[k], 100.0 * ph[8 + k] / (double)tp); fprintf(stderr, "\n");
 		}
 	}
+#endif
 	const char *trace_path = getenv("E264B_TRACE");
 	if (trace_path) {
 		FILE *f = fopen(trace_path, "w");

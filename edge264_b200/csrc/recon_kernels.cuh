@@ -71,7 +71,8 @@ __device__ __forceinline__ void reset_next_tickets(const PicJob &J) { if (blockI
 /* measurement only (replay with E264B_DIAG=1): how the blocks of each kernel kind land on the SMs —
  * [kind][sm]: blocks started, blocks of this kind resident right now, the maximum of that */
 __device__ unsigned g_diag_cnt[4][160], g_diag_cur[4][160], g_diag_max[4][160];
-/* -DE264_ROWS_TIMING (make variants): SM cycles the warps of e264_intra_rows_kernel spend per part of a macroblock step */
+/* -DE264_ROWS_TIMING / -DE264_INTER_TIMING (make variants): SM cycles the warps of e264_intra_rows_kernel spend per part
+ * of a macroblock step, or those of e264_inter4_kernel per part of a chunk */
 __device__ unsigned long long g_diag_phase[16];
 #ifdef E264_ROWS_TIMING
 #define RT_DECL unsigned rt_acc[8] = {0, 0, 0, 0, 0, 0, 0, 0}; unsigned rt_t = (unsigned)clock64();
@@ -81,6 +82,18 @@ __device__ unsigned long long g_diag_phase[16];
 #define RT_DECL
 #define RT_MARK(k)
 #define RT_FLUSH(base)
+#endif
+/* -DE264_INTER_TIMING (make variants): SM cycles the warps of e264_inter4_kernel spend per part of a chunk, all warps
+ * summed: 0 records + binning, 1 interpolation, 2 digest, 3 residual, 4 combine + store (a barrier's wait counts to the
+ * part in front of it) */
+#ifdef E264_INTER_TIMING
+#define IT_DECL unsigned long long it_acc[5] = {0, 0, 0, 0, 0}; long long it_t = clock64();
+#define IT_MARK(k) { const long long it_n = clock64(); it_acc[k] += (unsigned long long)(it_n - it_t); it_t = it_n; }
+#define IT_FLUSH if (lane == 0) { for (int it_k = 0; it_k < 5; it_k++) atomicAdd(&g_diag_phase[it_k], it_acc[it_k]); }
+#else
+#define IT_DECL
+#define IT_MARK(k)
+#define IT_FLUSH
 #endif
 /* measurement only: first-start / last-end timestamps of a launch, see e264b_replay */
 struct TraceScope {
@@ -140,9 +153,9 @@ __device__ __forceinline__ bool mbar_wait(void *bar, unsigned parity) {
 /* ------------------------------------------------------------------------------------------ */
 /* residual                                                                                     */
 /* ------------------------------------------------------------------------------------------ */
-/* 4x4 inverse transform of 16 levels at c (16-byte aligned) -> residual written to dst[y*dstride+x] */
+/* 4x4 inverse transform of 16 levels at c (16-byte aligned) -> residual o[y*4+x] in registers, saturated to int16 */
 static_assert(offsetof(E264SliceRec, scaling4x4) % 8 == 0 && sizeof(E264SliceRec) % 8 == 0, "idct4x4 loads a 4x4 scaling list as two 8-byte words");
-__device__ __noinline__ void idct4x4(const int16_t *c, bool have_levels, const uint8_t *scaling, int qp, bool dc_override, int dc, int16_t *dst, int dstride) {
+__device__ __forceinline__ void idct4x4_core(const int16_t *c, bool have_levels, const uint8_t *scaling, int qp, bool dc_override, int dc, int o[16]) {
 	int d[16];
 	if (have_levels) {
 		uint4 a = *(const uint4 *)c, b = *((const uint4 *)c + 1);   /* c points into the TMA-staged shared copy */
@@ -178,11 +191,20 @@ __device__ __noinline__ void idct4x4(const int16_t *c, bool have_levels, const u
 	for (int j = 0; j < 4; j++) {
 		int g0 = f[j] + f[8 + j], g1 = f[j] - f[8 + j];
 		int g2 = (f[4 + j] >> 1) - f[12 + j], g3 = f[4 + j] + (f[12 + j] >> 1);
-		dst[j] = (int16_t)sat16((g0 + g3 + 32) >> 6);
-		dst[dstride + j] = (int16_t)sat16((g1 + g2 + 32) >> 6);
-		dst[2 * dstride + j] = (int16_t)sat16((g1 - g2 + 32) >> 6);
-		dst[3 * dstride + j] = (int16_t)sat16((g0 - g3 + 32) >> 6);
+		o[j] = sat16((g0 + g3 + 32) >> 6);
+		o[4 + j] = sat16((g1 + g2 + 32) >> 6);
+		o[8 + j] = sat16((g1 - g2 + 32) >> 6);
+		o[12 + j] = sat16((g0 - g3 + 32) >> 6);
 	}
+}
+/* the same, residual written to dst[y*dstride+x] */
+__device__ __noinline__ void idct4x4(const int16_t *c, bool have_levels, const uint8_t *scaling, int qp, bool dc_override, int dc, int16_t *dst, int dstride) {
+	int o[16];
+	idct4x4_core(c, have_levels, scaling, qp, dc_override, dc, o);
+#pragma unroll
+	for (int y = 0; y < 4; y++)
+#pragma unroll
+		for (int x = 0; x < 4; x++) dst[y * dstride + x] = (int16_t)o[y * 4 + x];
 }
 
 /* one 8-point pass in the reference's int16 arithmetic (edge264_residual.c:250-296) */
@@ -195,6 +217,52 @@ __device__ __forceinline__ void idct8_1d(short a[8]) {
 	short f4 = (short)(e2 - e4), f5 = (short)((e3 >> 2) - e5), f6 = (short)(e0 - e6), f7 = (short)(e7 - (e1 >> 2));
 	a[0] = (short)(f0 + f7); a[1] = (short)(f2 + f5); a[2] = (short)(f4 + f3); a[3] = (short)(f6 + f1);
 	a[4] = (short)(f6 - f1); a[5] = (short)(f4 - f3); a[6] = (short)(f2 - f5); a[7] = (short)(f0 - f7);
+}
+
+/* luma of a macroblock with the 8x8 transform: lane (blk, k) = (lane >> 3, lane & 7) runs row k then column k of 8x8 block
+ * blk through the two passes; the residual of every coded 8x8 block goes to ws->res (luma y*16+x), the others are not
+ * written.  cf_luma: the macroblock's first luma level in the staged coefficient run. */
+__device__ __forceinline__ void residual_luma8x8(WarpSmem *ws, const E264MbRec *r, const E264SliceRec *sr, const int16_t *cf_luma, int lane) {
+	const unsigned coded = r->coded;
+	const int inter = r->kind == MBK_INTER, qpy = r->qp[0];
+	int blk = lane >> 3, k = lane & 7;
+	bool on = (coded >> (blk * 4)) & 1;
+	short a[8];
+	if (on) {
+		int idx = __popc(coded & 0x1111 & ((1u << (blk * 4)) - 1));
+		uint4 q = *(const uint4 *)(cf_luma + idx * 64 + k * 8);
+		short lv[8]; *(uint4 *)lv = q;
+		int div = qpy / 6, m = qpy - div * 6;
+		const uint8_t *sc = sr->scaling8x8[inter] + k * 8;
+#pragma unroll
+		for (int j = 0; j < 8; j++) {
+			int ls = sc[j] * norm8(m, k, j);
+			a[j] = div < 6 ? (short)sat16((lv[j] * ls + (1 << (5 - div))) >> (6 - div)) : (short)(lv[j] * (short)(ls << (div - 6)));
+		}
+		idct8_1d(a);
+#pragma unroll
+		for (int j = 0; j < 8; j++) ws->u.t8[blk * 64 + k * 8 + j] = a[j];
+	}
+	__syncwarp();
+	if (on) {
+#pragma unroll
+		for (int j = 0; j < 8; j++) a[j] = ws->u.t8[blk * 64 + j * 8 + k];
+		a[0] = (short)(a[0] + 32);
+		idct8_1d(a);
+		int x = (blk & 1) * 8 + k, y0 = (blk >> 1) * 8;
+#pragma unroll
+		for (int j = 0; j < 8; j++) ws->res[(y0 + j) * 16 + x] = (short)(a[j] >> 6);
+	}
+	__syncwarp();
+}
+
+/* scaled DC of chroma 4x4 block i of plane pl: the 2x2 transform of the plane's four DC levels at cdc (8.5.11) */
+__device__ __forceinline__ int chroma_dc(const int16_t *cdc, const E264MbRec *r, const E264SliceRec *sr, int inter, int pl, int i) {
+	const int a = cdc[4 * pl], b = cdc[4 * pl + 1], c = cdc[4 * pl + 2], d = cdc[4 * pl + 3];
+	const int f = i == 0 ? a + b + c + d : i == 1 ? a - b + c - d : i == 2 ? a + b - c - d : a - b - c + d;
+	const int qpc = r->qp[1 + pl];
+	const int ls = (sr->scaling4x4[1 + pl + inter * 3][0] * h264_norm4x4[qpc % 6][0]) << (qpc / 6);
+	return (f * ls) >> 5;
 }
 
 /* cf: this macroblock's coefficient run, staged in shared memory by the caller (cp.async.bulk) */
@@ -229,50 +297,12 @@ __device__ __noinline__ void residual_stage(WarpSmem *ws, const E264MbRec *r, co
 	cf += n_luma;
 	const bool any_cdc = (coded & (CODED_CB_DC | CODED_CR_DC)) != 0;
 	if (lane >= 16 && lane < 24) {
-		int pl = (lane - 16) >> 2, i = lane & 3, v = 0;
-		if (any_cdc) {
-			int a = cf[4 * pl], b = cf[4 * pl + 1], c = cf[4 * pl + 2], d = cf[4 * pl + 3];
-			int f = i == 0 ? a + b + c + d : i == 1 ? a - b + c - d : i == 2 ? a + b - c - d : a - b - c + d;
-			int qpc = r->qp[1 + pl];
-			int ls = (sr->scaling4x4[1 + pl + inter * 3][0] * h264_norm4x4[qpc % 6][0]) << (qpc / 6);
-			v = (f * ls) >> 5;
-		}
-		ws->dc[16 + pl * 4 + i] = v;
+		const int pl = (lane - 16) >> 2, i = lane & 3;
+		ws->dc[16 + pl * 4 + i] = any_cdc ? chroma_dc(cf, r, sr, inter, pl, i) : 0;
 	}
 	if (any_cdc) cf += 8;
 	__syncwarp();
-	/* --- luma --- */
-	if (r->flags & MBF_T8x8) {
-		int blk = lane >> 3, k = lane & 7;
-		bool on = (coded >> (blk * 4)) & 1;
-		short a[8];
-		if (on) {
-			int idx = __popc(coded & 0x1111 & ((1u << (blk * 4)) - 1));
-			uint4 q = *(const uint4 *)(cf_luma + idx * 64 + k * 8);
-			short lv[8]; *(uint4 *)lv = q;
-			int div = qpy / 6, m = qpy - div * 6;
-			const uint8_t *sc = sr->scaling8x8[inter] + k * 8;
-#pragma unroll
-			for (int j = 0; j < 8; j++) {
-				int ls = sc[j] * norm8(m, k, j);
-				a[j] = div < 6 ? (short)sat16((lv[j] * ls + (1 << (5 - div))) >> (6 - div)) : (short)(lv[j] * (short)(ls << (div - 6)));
-			}
-			idct8_1d(a);
-#pragma unroll
-			for (int j = 0; j < 8; j++) ws->u.t8[blk * 64 + k * 8 + j] = a[j];
-		}
-		__syncwarp();
-		if (on) {
-#pragma unroll
-			for (int j = 0; j < 8; j++) a[j] = ws->u.t8[blk * 64 + j * 8 + k];
-			a[0] = (short)(a[0] + 32);
-			idct8_1d(a);
-			int x = (blk & 1) * 8 + k, y0 = (blk >> 1) * 8;
-#pragma unroll
-			for (int j = 0; j < 8; j++) ws->res[(y0 + j) * 16 + x] = (short)(a[j] >> 6);
-		}
-		__syncwarp();
-	}
+	if (r->flags & MBF_T8x8) residual_luma8x8(ws, r, sr, cf_luma, lane);
 	/* --- 4x4 blocks: luma on lanes 0..15 (unless the macroblock uses the 8x8 transform) and chroma AC (+DC) on lanes
 	 * 16..23 go through ONE call of the transform --- */
 	{
